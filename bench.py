@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 pairwise string-similarity hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): char-trigram TF-IDF top-10, company-names self-match,
 n = 100 000 -- on the reference's own data/company_names.json (shipped as a test fixture under
@@ -18,6 +18,10 @@ N > 1 (torchrun, one rank per GPU, NCCL): weak scaling.  The to_list grows to N 
 row-sharded (rank r owns block r); the from_list stays the first block (100 000 names), scored
 against all shards with the global diagonal excluded -- i.e. one from-row-block of the N*100k
 self-match.  Per-GPU work is fixed; one all-reduce (df) + one all-gather (top-k) per step.
+
+--steps sets the number of timed steps of every leg and sub-record.  --dump-outputs DIR writes what the last timed step
+of the headline leg returned (top-10 indices and scores per from-row) as DIR/<name>.npy in float64, so that the
+outputs of two builds can be compared on identical inputs.
 
 Prints ONE JSON line on rank 0 (see the repository README / DESIGN.md for the keys).
 """
@@ -53,6 +57,7 @@ def parse():
     ap.add_argument("--skip", default="", help="comma list of sub-records to skip: c3,c4,c5,e2e")
     ap.add_argument("--c5-n", type=int, default=1_000_000, help="rows per list of the c5 sub-record")
     ap.add_argument("--synthetic", action="store_true", help="force the synthetic stand-in data")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's top-k indices / scores as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -230,6 +235,25 @@ def hbm_peak():
     return {}, 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (rows x k) array as out_dir/<name>.npy in float64.  Above DUMP_LIMIT_BYTES in all, the same fixed,
+    seeded sample of rows is written for every array, and the sampled row numbers as rows.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = int(n * (DUMP_LIMIT_BYTES - (1 << 16)) // (total + 8 * n))      # 64 KiB left for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def timed(fn, warmup, steps, sync, flush=None):
     """Device time of fn() per call (CUDA events on the current stream), after `warmup` untimed calls."""
     import torch
@@ -274,7 +298,7 @@ def load_names(args, rank, world):
 
 
 # ---- sub-records -------------------------------------------------------------------------------------
-def sub_c3(dev, local_rank, sync, flush):
+def sub_c3(dev, local_rank, sync, flush, steps):
     """BASELINE configs[2]: all-pairs edit distance on movie_titles (Netflix 6 172 x IMDB 80 852), per-row best match.
     Device-timed from staged blobs (EditQueries / EditTargets) to the arg-best arrays; integer-ALU roofline against the
     INT32 issue rate measured by pfz_int_alu_probe in this run."""
@@ -305,7 +329,7 @@ def sub_c3(dev, local_rank, sync, flush):
         res = {}
         def run():
             res["r"] = editdist.edit_argbest_staged(Q, T, metric)
-        ms = timed(run, 2, 5, sync, flush)
+        ms = timed(run, 2, steps, sync, flush)
         t = float(np.median(ms)) * 1e-3
         alg_ops = word_steps32 * ops
         out[key] = {"ms": t * 1e3, "ms_each": [round(x, 3) for x in ms], "pairs_per_s": pairs / t, "gcups": cells / t / 1e9,
@@ -319,7 +343,7 @@ def sub_c3(dev, local_rank, sync, flush):
     return out
 
 
-def sub_c4(dev, local_rank, sync, flush, peaks):
+def sub_c4(dev, local_rank, sync, flush, peaks, steps):
     """BASELINE configs[3]: dense cosine top-10, 100k x 100k x 768 random unit vectors (bf16 in, fp32 accumulate)."""
     import torch
     from polyfuzz_b200 import dense
@@ -329,7 +353,7 @@ def sub_c4(dev, local_rank, sync, flush, peaks):
     x, _ = dense.to_bf16_rows(X, True); y, _ = dense.to_bf16_rows(Y, True)
     del X, Y
     sampler = ClockSampler(local_rank)
-    ms = timed(lambda: dense.dense_topk(x, y, k, 0.0), 3, 10, sync, flush)
+    ms = timed(lambda: dense.dense_topk(x, y, k, 0.0), 3, steps, sync, flush)
     clocks = sampler.stop()
     t = float(np.median(ms)) * 1e-3
     flops = 2.0 * n * n * d
@@ -373,7 +397,7 @@ def sub_c5(args, dev, rank, local_rank, world, comm, barrier, flush, peak):
     if sampler:
         sampler.recording = True
     ms = []
-    for _ in range(3):
+    for _ in range(args.steps):
         flush.zero_(); barrier()
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
         e0.record(); step(True); e1.record()
@@ -485,6 +509,8 @@ def run_b200(args):
     k2_ms = [a.elapsed_time(b) for a, b in k2_events]
     k1_ms = [a.elapsed_time(b) for a, b in k1_events]
 
+    if args.dump_outputs and rank == 0:
+        outputs = {"top_idx": result["idx"].cpu().numpy(), "top_val": result["val"].cpu().numpy()}
     keep = {k: result[k] for k in ("vec", "csr", "index")}
     result.clear(); result.update(keep)
     gc.enable(); gc.collect(); gc.disable()
@@ -498,7 +524,7 @@ def run_b200(args):
         return m.match(from_list)
 
     e2e_ms = []
-    e2e_steps = max(3, args.steps)
+    e2e_steps = args.steps
     for it in range(2 + e2e_steps):
         flush.zero_()
         barrier()
@@ -518,9 +544,9 @@ def run_b200(args):
     # ---- sub-records (other BASELINE configs), every one with its own clock record ----------------
     subs = {}
     if world == 1 and "c3" not in skip:
-        subs["c3"] = sub_c3(dev, local_rank, torch.cuda.synchronize, flush)
+        subs["c3"] = sub_c3(dev, local_rank, torch.cuda.synchronize, flush, args.steps)
     if world == 1 and "c4" not in skip:
-        subs["c4"] = sub_c4(dev, local_rank, torch.cuda.synchronize, flush, peaks)
+        subs["c4"] = sub_c4(dev, local_rank, torch.cuda.synchronize, flush, peaks, args.steps)
     if "c5" not in skip:
         keep_main = dict(result)
         subs["c5"] = sub_c5(args, dev, rank, local_rank, world, comm, barrier, flush, peak)
@@ -603,6 +629,8 @@ def run_b200(args):
             "step_outliers_over_5pct": int(sum(1 for x in step_ms if x > 1.05 * med)),
             "k1_ms_avg": float(np.mean(k1_ms)) if k1_ms else None, "k2_ms_avg": k2_avg_ms}
     line.update(subs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,16 +1,31 @@
 """Import shim that lets the UNMODIFIED reference (/root/reference) be imported in the build
 container, where its optional third-party deps (rapidfuzz, matplotlib, seaborn) are absent.
-TEST INFRASTRUCTURE -- used only by tests/golden/make_golden.py and by CPU tests that are skipped
-when /root/reference is not present (it does not exist on the GPU box)."""
+TEST INFRASTRUCTURE -- used by tests/golden/make_golden.py, and by the GPU tests that run the reference's
+orchestrator from the copy stage() makes (they skip where there is none)."""
 import os
 import sys
 import types
 
 REFERENCE_ROOT = os.environ.get("PFZ_REFERENCE_ROOT", "/root/reference")
+# git-ignored copy of the reference's package, made by stage(): machines that only receive the working tree import it from here
+STAGED_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def available() -> bool:
     return os.path.isdir(os.path.join(REFERENCE_ROOT, "polyfuzz"))
+
+
+def stage() -> bool:
+    """Copy the reference's pure-Python package (REFERENCE_ROOT/polyfuzz) to STAGED_ROOT/polyfuzz.  Returns False and
+    changes nothing when the reference is not readable here."""
+    src = os.path.join(REFERENCE_ROOT, "polyfuzz")
+    if not os.path.isdir(src) or os.path.abspath(REFERENCE_ROOT) == STAGED_ROOT:
+        return False
+    import shutil
+    dst = os.path.join(STAGED_ROOT, "polyfuzz")
+    shutil.rmtree(dst, ignore_errors=True)
+    shutil.copytree(src, dst, ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
+    return True
 
 
 def install():

@@ -1,5 +1,5 @@
-"""Drop-in test with the UNMODIFIED reference orchestrator (polyfuzz.PolyFuzz installed from /root/reference
-into baseline/_ref, which travels to the GPU box): the B200 matchers are handed to PolyFuzz.match / fit /
+"""Drop-in test with the UNMODIFIED reference orchestrator (polyfuzz.PolyFuzz, copied into oracle/_ref by build()
+when a reference checkout is readable): the B200 matchers are handed to PolyFuzz.match / fit /
 transform / group exactly as the reference's own tests do (tests/test_polyfuzz.py:40-146)."""
 import os
 import sys
@@ -10,7 +10,7 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 FROM = ["apple", "apples", "appl", "recal", "house", "similarity"]
 TO = ["apple", "apples", "mouse"]
 
@@ -18,7 +18,7 @@ TO = ["apple", "apples", "mouse"]
 @pytest.fixture(scope="module")
 def PolyFuzz():
     if not os.path.isdir(os.path.join(REF, "polyfuzz")):
-        pytest.skip("baseline/_ref (pip install of the reference) not present")
+        pytest.skip("oracle/_ref (the reference's polyfuzz package, copied by build()) not present")
     os.environ["PFZ_REFERENCE_ROOT"] = REF
     from oracle import ref_shim
     ref_shim.REFERENCE_ROOT = REF

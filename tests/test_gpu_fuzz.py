@@ -98,9 +98,9 @@ def test_matchers_default_to_wratio_like_the_reference():
 def test_string_shortcut_through_the_unmodified_orchestrator():
     """polyfuzz_b200.install() + PolyFuzz("EditDistance") (polyfuzz/polyfuzz.py:128-130: RapidFuzz() -> WRatio) reproduces
     rapidfuzz's published extractOne answer through the reference's own orchestrator."""
-    ref = os.path.join(ROOT, "baseline", "_ref")
+    ref = os.path.join(ROOT, "oracle", "_ref")
     if not os.path.isdir(os.path.join(ref, "polyfuzz")):
-        pytest.skip("baseline/_ref (pip install of the reference) not present")
+        pytest.skip("oracle/_ref (the reference's polyfuzz package, copied by build()) not present")
     os.environ["PFZ_REFERENCE_ROOT"] = ref
     from oracle import ref_shim
     ref_shim.REFERENCE_ROOT = ref
